@@ -19,6 +19,9 @@ V = 10M, and 100M - the north-star size - when N = 8).
                bytes (SURVEY.md 8d) / CUDA-event time, L2 flushed between launches, vs MEASURED_PEAKS.json hbm_gbs
   cpu_baseline the CPU oracle port of the same step on a bounded sample (rank 0, N = 1)
 
+`--dump-outputs DIR` writes what the last timed train_step returned (loss, predictions) as DIR/<name>.npy on rank 0;
+the batches and the initial weights are seeded, so the same arguments give the same inputs on every run.
+
 `--impl reference` times the CPU oracle port (TensorFlow, hence the real reference, cannot be installed in this
 image: DESIGN.md) with the host threads it runs fastest with, for exactly --steps / --warmup steps (capped at 64).
 """
@@ -62,7 +65,43 @@ def parse():
   ap.add_argument('--no-cpu-baseline', action='store_true')
   ap.add_argument('--no-extras', action='store_true', help='skip the optimizer / file / C3 lines (quick runs)')
   ap.add_argument('--kernel-iters', type=int, default=30)
+  ap.add_argument('--dump-outputs', default='', metavar='DIR',
+                  help='after the timed steps, write what the last timed train_step returned (loss, predictions) '
+                       'as DIR/<name>.npy, so that two builds can be compared output for output')
   return ap.parse_args()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, outputs):
+  """outputs: name -> tensor, array, or a list / dict of them.  Each leaf is written as DIR/<name>.npy in float32
+  (float64 stays float64).  If the leaves exceed DUMP_BYTES in all, each is replaced by a fixed, seeded sample of
+  its flattened elements (sorted indices), the same sample on every run."""
+  import torch
+  leaves = {}
+
+  def walk(name, x):
+    if isinstance(x, dict):
+      for k in sorted(x):
+        walk('%s_%s' % (name, k), x[k])
+    elif isinstance(x, (list, tuple)):
+      for i, v in enumerate(x):
+        walk('%s_%d' % (name, i), v)
+    elif x is not None:
+      t = torch.as_tensor(x).detach()
+      leaves[name] = (t.double() if t.dtype == torch.float64 else t.float()).cpu().numpy()
+
+  for name, x in outputs.items():
+    walk(name, x)
+  total = sum(a.nbytes for a in leaves.values())
+  os.makedirs(out_dir, exist_ok=True)
+  for name, a in leaves.items():
+    if total > DUMP_BYTES:
+      keep = max(1, int(a.size * DUMP_BYTES // total))
+      idx = np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))
+      a = a.reshape(-1)[idx]
+    np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def peaks():
@@ -322,17 +361,18 @@ def main():
     return devb[(i + 1) % n_rot][0] if (ep and i + 1 < n) else None
 
   def timed_resident(est, steps, warm):
-    """device-resident throughput: CUDA events around `steps` train_step calls"""
+    """device-resident throughput: CUDA events around `steps` train_step calls; also returns what the last of them
+    returned (under CUDA-graph replay these are the graph's output buffers, rewritten by the next step)"""
     for i in range(warm):
       est.trainer.train_step(*devb[i % n_rot], next_features=nxt(i, warm))
     barrier()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     for i in range(steps):
-      loss, _ = est.trainer.train_step(*devb[i % n_rot], next_features=nxt(i, steps))
+      loss, probs = est.trainer.train_step(*devb[i % n_rot], next_features=nxt(i, steps))
     ev1.record()
     barrier()
-    return max_over_ranks(ev0.elapsed_time(ev1)), float(loss)
+    return max_over_ranks(ev0.elapsed_time(ev1)), loss, probs
 
   def timed_train(est, input_fn, steps, warm):
     """EasyRecEstimator.train end to end: reader thread -> pinned staging -> H2D -> step -> loss D2H, per step"""
@@ -355,7 +395,10 @@ def main():
     est.trainer.train_step(*devb[i % n_rot], next_features=nxt(i, W))
   barrier()
   sampler.mark()
-  ms, final_loss = timed_resident(est, args.steps, 0)
+  ms, last_loss, last_probs = timed_resident(est, args.steps, 0)
+  final_loss = float(last_loss)
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, {'loss': last_loss, 'probs': last_probs})
   value = world * B * args.steps / (ms / 1000.0)
   per_step_launches = getattr(est.trainer, 'launches_per_step', None)
   if per_step_launches is None:   # eager run: count the launches of one step
@@ -440,7 +483,7 @@ def main():
                           'gpu_launches_per_step': int(per_step_launches)})
         continue
       e = build(o)
-      m, _ = timed_resident(e, o_steps, o_warm + 3)
+      m, _, _ = timed_resident(e, o_steps, o_warm + 3)
       row = {'optimizer': o, 'value': B * o_steps / (m / 1000.0), 'ms_per_step': m / o_steps,
              'cuda_graph': graph and e.trainer._graph is not None,
              'gpu_launches_per_step': int(getattr(e.trainer, 'launches_per_step', 0) or 0)}
@@ -546,10 +589,12 @@ def run_c4(args, rank, world, dev, ep, graph, barrier, max_over_ranks):
   ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
   ev0.record()
   for i in range(steps):
-    loss, _ = est.trainer.train_step(*devb[i % n_rot], next_features=nxt(i, steps))
+    loss, probs = est.trainer.train_step(*devb[i % n_rot], next_features=nxt(i, steps))
   ev1.record()
   barrier()
   ms = max_over_ranks(ev0.elapsed_time(ev1))
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, {'loss': loss, 'probs': probs})
   launches = int(lib.er_launch_count() - n0)
   if getattr(est.trainer, 'launches_per_step', None):
     launches = int(est.trainer.launches_per_step) * steps

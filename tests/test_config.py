@@ -1,19 +1,20 @@
 """CPU: pipeline-config loading (runtime proto2 schema, text_format) and config -> model plan.
 
-When the reference checkout is mounted (/root/reference, build container only) the subset schema is
-cross-checked field by field against the reference's protos and every reference sample config is parsed;
-on the GPU box those cases skip and the in-repo config texts below still run."""
-import glob
+The subset schema is cross-checked field by field against a record of the reference's protos, and the reference's
+sample configs, stored under tests/golden (reference_configs.py), are parsed and built."""
 import os
+import sys
 
 import pytest
 import torch
 
 from easyrec_b200 import builder
-from easyrec_b200.config import config_util, proto_loader
+from easyrec_b200.config import config_util
 
-REF = '/root/reference'
-HAVE_REF = os.path.isdir(os.path.join(REF, 'easy_rec/python/protos'))
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden'))
+import reference_configs  # noqa: E402
+
+REF_CONFIGS = reference_configs.load()
 
 MINI = b'''
 model_dir: "/tmp/m"
@@ -61,27 +62,22 @@ def test_config_to_table_plan_and_schedule():
   assert model.l2_of('dnn.layers.0.bias', None) == 0.0
 
 
-@pytest.mark.skipif(not HAVE_REF, reason='reference checkout not mounted')
 def test_subset_schema_is_consistent_with_reference_protos():
-  import sys
   sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'tools'))
   import check_subset_schema
-  assert check_subset_schema.check(os.path.join(REF, 'easy_rec/python/protos')) == []
+  assert check_subset_schema.check(reference_configs.record()['schema']) == []
 
 
-@pytest.mark.skipif(not HAVE_REF, reason='reference checkout not mounted')
 def test_every_reference_sample_config_parses():
-  full = proto_loader.load_schema(sorted(glob.glob(os.path.join(REF, 'easy_rec/python/protos/*.proto'))),
-                                  virtual_name='full_ref.proto')
-  paths = sorted(glob.glob(os.path.join(REF, 'samples/model_config/*.config'))) + \
-      sorted(glob.glob(os.path.join(REF, 'examples/configs/*.config')))
-  assert len(paths) > 200
-  for p in paths:
-    config_util.get_configs_from_pipeline_file(p, schema=full)  # strict: complete schema
-    config_util.get_configs_from_pipeline_file(p)               # subset schema, unknown fields skipped
+  """every config parses under the subset schema (unknown fields skipped), and every field it keeps is one the
+  reference's complete schema parsed out of the same config (strictly, when the record was written)."""
+  full = reference_configs.recorded_field_paths()
+  assert len(REF_CONFIGS) > 200 and set(full) == set(REF_CONFIGS)
+  for p, text in REF_CONFIGS.items():
+    kept = reference_configs.field_paths(config_util.get_configs_from_pipeline_file(text))
+    assert kept <= full[p], (p, sorted(kept - full[p]))
 
 
-@pytest.mark.skipif(not HAVE_REF, reason='reference checkout not mounted')
 @pytest.mark.parametrize('rel', ['examples/configs/deepfm_on_criteo.config', 'samples/model_config/din_on_taobao.config',
                                  'samples/model_config/dcn_on_taobao.config', 'samples/model_config/dssm_on_taobao.config',
                                  'samples/model_config/mmoe_on_taobao.config',
@@ -97,7 +93,7 @@ def test_every_reference_sample_config_parses():
                                  'examples/configs/wide_and_deep_backbone_on_movielens.config'])
 def test_baseline_model_families_build_from_unmodified_reference_configs(rel, monkeypatch):
   monkeypatch.setenv('ER_PLAN_ONLY', '1')   # the plan is what is checked: the 10M-row criteo tables are not randomised
-  cfg = config_util.get_configs_from_pipeline_file(os.path.join(REF, rel))
+  cfg = config_util.get_configs_from_pipeline_file(REF_CONFIGS[rel])
   il, model, opt = builder.build_model(cfg, 16, 'cpu', cpu_generator=torch.Generator().manual_seed(0))
   assert sum(p.numel() for p in model.parameters()) > 1000
   assert all(a.n_rows > 0 for a in il.arenas.values())
@@ -181,7 +177,6 @@ def test_cross_layer_variants_have_the_keras_parameter_shapes():
     BB.Cross(12, {'diag_scale': -1.0})
 
 
-@pytest.mark.skipif(not HAVE_REF, reason='reference checkout not mounted')
 def test_reference_criteo_config_reads_kaggle_format_lines(tmp_path):
   """examples/configs/deepfm_on_criteo.config as it is (STRING categorical fields with hash_bucket_size, FLOAT
   integer counts, empty cells) over lines in the Criteo Kaggle layout (examples/data/criteo/process_criteo_kaggle.py):
@@ -191,7 +186,7 @@ def test_reference_criteo_config_reads_kaggle_format_lines(tmp_path):
   from easyrec_b200 import _lib
   from easyrec_b200.input import readers
   from oracle import oracle as O
-  cfg = config_util.get_configs_from_pipeline_file(os.path.join(REF, 'examples/configs/deepfm_on_criteo.config'))
+  cfg = config_util.get_configs_from_pipeline_file(REF_CONFIGS['examples/configs/deepfm_on_criteo.config'])
   cfg = config_util.edit_config(cfg, {'data_config.batch_size': 8})
   il, model, _ = builder.build_model(cfg, 8, 'cpu', cpu_generator=torch.Generator().manual_seed(0))
   rng = np.random.default_rng(3)
@@ -232,23 +227,21 @@ def test_optimizers_without_a_fused_row_rule_are_refused():
         b'train_config { optimizer_config { ftrl_optimizer { } } }'))
 
 
-@pytest.mark.skipif(not HAVE_REF, reason='reference checkout not mounted')
 @pytest.mark.parametrize('rel,why', [
     ('samples/model_config/multi_tower_backbone_on_taobao.config', 'losses'),           # F1-reweighted + pairwise
     ('samples/model_config/deepfm_multi_cls_on_avazu_ctr.config', None),
     ('samples/model_config/wide_and_deep_two_opti.config', None),
     ('samples/model_config/taobao_fg_ev.config', 'ev_params')])
 def test_configs_that_need_unimplemented_training_semantics_are_refused(rel, why):
-  cfg = config_util.get_configs_from_pipeline_file(os.path.join(REF, rel))
+  cfg = config_util.get_configs_from_pipeline_file(REF_CONFIGS[rel])
   with pytest.raises((NotImplementedError, KeyError, ValueError)) as e:
     builder.build_model(cfg, 16, 'cpu', cpu_generator=torch.Generator().manual_seed(0))
   if why:
     assert why in str(e.value)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason='reference checkout not mounted')
 def test_the_reference_regression_sample_builds_with_its_l2_loss():
-  cfg = config_util.get_configs_from_pipeline_file(os.path.join(REF, 'samples/model_config/deepfm_combo_on_avazu_reg.config'))
+  cfg = config_util.get_configs_from_pipeline_file(REF_CONFIGS['samples/model_config/deepfm_combo_on_avazu_reg.config'])
   os.environ['ER_PLAN_ONLY'] = '1'
   try:
     _, model, _ = builder.build_model(cfg, 16, 'cpu', cpu_generator=torch.Generator().manual_seed(0))
@@ -330,7 +323,6 @@ def test_every_config_embedded_in_the_gpu_tests_builds_without_a_gpu():
   assert n >= 10
 
 
-@pytest.mark.skipif(not HAVE_REF, reason='reference checkout not mounted')
 def test_reference_avazu_combo_config_reads_synthetic_lines(tmp_path):
   """samples/model_config/deepfm_combo_on_avazu_ctr.config, the DeepFM config of the reference's own train tests
   (STRING hashed ids, bucketized RawFeatures, a ComboFeature): it builds unmodified and its reader turns text lines
@@ -339,7 +331,7 @@ def test_reference_avazu_combo_config_reads_synthetic_lines(tmp_path):
   from easyrec_b200 import _lib
   from easyrec_b200.input import readers
   from oracle import oracle as O
-  cfg = config_util.get_configs_from_pipeline_file(os.path.join(REF, 'samples/model_config/deepfm_combo_on_avazu_ctr.config'))
+  cfg = config_util.get_configs_from_pipeline_file(REF_CONFIGS['samples/model_config/deepfm_combo_on_avazu_ctr.config'])
   cfg = config_util.edit_config(cfg, {'data_config.batch_size': 8})
   il, model, _ = builder.build_model(cfg, 8, 'cpu', cpu_generator=torch.Generator().manual_seed(0))
   types = builder.input_field_types(cfg)
@@ -408,39 +400,26 @@ def test_non_binary_task_towers_are_refused():
   builder.check_scope(config_util.get_configs_from_pipeline_file(G.MMOE_CFG.encode()))
 
 
-@pytest.mark.skipif(not HAVE_REF, reason='reference checkout not mounted')
 def test_no_model_or_optimizer_field_is_silently_dropped_for_configs_that_build(monkeypatch):
   """The subset schema skips fields it does not know.  For every reference sample config that BUILDS here, parse it
   with the reference's full schema as well and diff the set fields: anything under model_config, the optimizer, the
   label / input-field declarations that the subset dropped would mean training a different model in silence.
-  (Control plane - export, kafka / odps inputs, extra eval metrics - may be dropped.)"""
-  full = proto_loader.load_schema(sorted(glob.glob(os.path.join(REF, 'easy_rec/python/protos/*.proto'))),
-                                  virtual_name='full_ref2.proto')
+  (Control plane - export, kafka / odps inputs, extra eval metrics - may be dropped.)  The full schema's field paths
+  are the ones recorded with the stored configs."""
+  full = reference_configs.recorded_field_paths()
   # (only the plan matters here: the 10M-row tables of the criteo configs are allocated but not randomised)
   monkeypatch.setenv('ER_PLAN_ONLY', '1')
-
-  def walk(msg, prefix, out):
-    for fd, v in msg.ListFields():
-      p = prefix + '.' + fd.name
-      out.add(p)
-      if fd.type == fd.TYPE_MESSAGE and not fd.message_type.GetOptions().map_entry:
-        for it in (list(v) if builder._is_repeated(fd) else [v]):
-          walk(it, p, out)
   guarded = ('.model_config', '.train_config.optimizer_config', '.train_config.gradient_clipping_by_norm',
              '.data_config.input_fields', '.data_config.label_fields', '.data_config.separator', '.data_config.sample_weight')
-  paths = sorted(glob.glob(os.path.join(REF, 'samples/model_config/*.config'))) + \
-      sorted(glob.glob(os.path.join(REF, 'examples/configs/*.config')))
   built, dropped = 0, {}
-  for p in paths:
+  for p, text in REF_CONFIGS.items():
     try:
-      cfg = config_util.get_configs_from_pipeline_file(p)
+      cfg = config_util.get_configs_from_pipeline_file(text)
       builder.build_model(cfg, 4, 'cpu', cpu_generator=torch.Generator().manual_seed(0))
     except (NotImplementedError, ValueError, KeyError, AssertionError):
       continue          # refused loudly: fine
     built += 1
-    a, b = set(), set()
-    walk(config_util.get_configs_from_pipeline_file(p, schema=full), '', a)
-    walk(cfg, '', b)
+    a, b = full[p], reference_configs.field_paths(cfg)
     bad = sorted(f for f in a - b if f.startswith(guarded))
     if bad:
       dropped[os.path.basename(p)] = bad

@@ -7,6 +7,7 @@
   * model_class "DLRM" (model/dlrm.py:38-73): the reference's own EmbeddingParallel sample config builds, and the
     interaction equals the einsum / upper-triangle restatement of the reference body."""
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -125,10 +126,10 @@ def test_dlrm_interaction_matches_the_reference_body(itself, with_dense, interac
 
 def test_reference_dlrm_ep_config_builds(monkeypatch):
   """the reference's own EmbeddingParallel test config (model_class DLRM over the packed Parquet criteo form)"""
-  path = '/root/reference/samples/model_config/dlrm_on_criteo_parquet_ep.config'
-  if not os.path.exists(path):
-    pytest.skip('reference tree not mounted')
-  cfg = config_util.get_configs_from_pipeline_file(path)
+  sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden'))
+  import reference_configs
+  cfg = config_util.get_configs_from_pipeline_file(
+      reference_configs.load()['samples/model_config/dlrm_on_criteo_parquet_ep.config'])
   monkeypatch.setenv('ER_PLAN_ONLY', '1')   # (a 10M-row table: the plan is what is checked)
   il, model, opt = builder.build_model(cfg, 64, 'cpu', cpu_generator=torch.Generator().manual_seed(0))
   assert type(model).__name__ == 'DLRM' and builder.embedding_parallel(cfg)

@@ -1,9 +1,9 @@
 """CPU, kernel doubles: every reference sample config that the scope check accepts (and whose tables are small enough to
 materialise here) is built through EasyRecEstimator, trains two steps on a DummyInput batch and evaluates its
 eval_config.metrics_set - the reference's own train_eval tests are exit-code smoke runs over the same files
-(easy_rec/python/test/train_eval_test.py).  Needs /root/reference (skipped elsewhere, e.g. on the GPU box)."""
-import glob
+(easy_rec/python/test/train_eval_test.py).  The configs are the ones stored under tests/golden (reference_configs.py)."""
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -14,20 +14,18 @@ from easyrec_b200 import builder
 from easyrec_b200.config import config_util
 from easyrec_b200.input import readers
 
-REF = '/root/reference'
-PATHS = sorted(glob.glob(os.path.join(REF, 'samples/model_config/*.config'))) + \
-    sorted(glob.glob(os.path.join(REF, 'examples/configs/*.config')))
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden'))
+import reference_configs  # noqa: E402
 
 
-@pytest.mark.skipif(not PATHS, reason='reference checkout not mounted')
 @pytest.mark.timeout(900)
 def test_every_accepted_small_reference_config_trains_and_evaluates(monkeypatch):
   from easyrec_b200.estimator import EasyRecEstimator
   host_doubles.install_all(monkeypatch.setattr)
   trained, failed = [], {}
-  for p in PATHS:
+  for p, text in reference_configs.load().items():
     try:
-      cfg = config_util.get_configs_from_pipeline_file(p)
+      cfg = config_util.get_configs_from_pipeline_file(text)
       builder.check_scope(cfg)
       builder.feature_specs(cfg)
     except Exception:
