@@ -267,9 +267,9 @@ model_config { model_class: "MultiTaskModel"
              keras_layer { class_name: "MMoE" mmoe { num_task: 3 num_expert: 4 expert_mlp { hidden_units: [128, 64] } } } }
   }
   model_params { l2_regularization: 1e-6
-    task_towers { tower_name: "t0" label_name: "l0" mlp { hidden_units: [64] } }
-    task_towers { tower_name: "t1" label_name: "l1" mlp { hidden_units: [64] } }
-    task_towers { tower_name: "t2" label_name: "l2" mlp { hidden_units: [64] } } }
+    task_towers { tower_name: "t0" label_name: "l0" dnn { hidden_units: [64] } }
+    task_towers { tower_name: "t1" label_name: "l1" dnn { hidden_units: [64] } }
+    task_towers { tower_name: "t2" label_name: "l2" dnn { hidden_units: [64] } } }
   embedding_regularization: 1e-6 }
 ''' % ('train_distribute: EmbeddingParallelStrategy' if embedding_parallel else '', lr, batch_size, fields, feats,
        names)).encode()

@@ -1,13 +1,9 @@
-"""GPU parity at the BASELINE.json config shapes and through the layer glue (not only kernel by kernel):
+"""GPU parity through the layer glue (not only kernel by kernel): TensorFlow's SafeEmbeddingLookupSparseTest case
+table (invalid ids, empty rows, non-positive weights under mean) replayed on the KERNEL through a TagFeature group of
+InputLayer - lookup and the backward row update.
 
-  * C3 = DIN at its real shape (batch 4096, two histories of 50 steps, 1M-row item table, attention MLP
-    [128, 64, 32, 1]): the logits of the config-built MultiTowerDIN against a plain torch restatement of
-    layers/sequence_feature_layer.py:150-189 + model/multi_tower_din.py:62-97 whose table rows come from the ORACLE's
-    hashing, <= 1e-4;
-  * a C5-shaped multi-task model (MMoE over a DCN-style backbone: Cross x 3 + MLP, 3 task towers, batch 16384, dim 32
-    features) trains through the config path and its mixture equals the oracle's restatement of layers/mmoe.py:62-83;
-  * TensorFlow's SafeEmbeddingLookupSparseTest case table (invalid ids, empty rows, non-positive weights under mean)
-    replayed on the KERNEL through a TagFeature group of InputLayer - lookup and the backward row update.
+The training steps of the BASELINE.json configs C3, C4 and C5 at config shape are compared with float64 in
+test_gpu_config_step_parity.py.
 """
 import json
 import os
@@ -16,137 +12,12 @@ import numpy as np
 import pytest
 import torch
 
-from easyrec_b200 import _lib, builder, workloads
+from easyrec_b200 import builder
 from easyrec_b200.config import config_util
-from easyrec_b200.estimator import EasyRecEstimator
-from easyrec_b200.trainer import Trainer
-from oracle import oracle as O
 
 pytestmark = pytest.mark.gpu
 DEV = 'cuda:0'
 KATS = json.load(open(os.path.join(os.path.dirname(__file__), 'golden', 'reference_kats.json')))
-
-
-def _bn(x):
-  mu, var = x.mean(0), ((x - x.mean(0))**2).mean(0)
-  return (x - mu) / torch.sqrt(var + 1e-3)
-
-
-def _dnn(mod, x):
-  for lay in mod.layers:
-    x = x @ lay.kernel + lay.bias
-    if lay.use_bn:
-      x = _bn(x) * lay.gamma + lay.beta
-    if lay.relu:
-      x = torch.relu(x)
-  return x
-
-
-def test_din_c3_logits_match_the_torch_restatement_at_config_shape():
-  torch.backends.cuda.matmul.allow_tf32 = False
-  B, T, V = 4096, 50, 1_000_000
-  est = EasyRecEstimator(workloads.c3_config_text(B, V, T), device=DEV, seed=3, default_seq_len=T)
-  il, model = est.input_layer, est.model
-  f, _ = workloads.c3_batch(B, T, 9, V)
-  feats = {'sparse_fea': f['sparse_fea'].to(DEV), 'dense_fea': f['dense_fea'].to(DEV),
-           'seq_fea': {k: (a.to(DEV), b.to(DEV)) for k, (a, b) in f['seq_fea'].items()}}
-  model.train()
-  logits = model(feats).detach()
-  arena = il.arenas[16]
-  W = arena.weight.detach()
-
-  def table(name):
-    off, n, _ = arena.tables[name]
-    return W[off:off + n]
-
-  def hashed(v, nb):   # the oracle's as_string + Fingerprint64 % buckets
-    rows, _ = O.bucketize(np.ascontiguousarray(v.reshape(-1)), 0, nb, 0)
-    return torch.from_numpy(rows.reshape(v.shape)).to(DEV)
-  ids = f['sparse_fea'].numpy().reshape(4, B)
-  age = torch.from_numpy(np.where((ids[1] < 0) | (ids[1] >= 100), 0, ids[1])).to(DEV)
-  user = torch.cat([table('user_id_embedding')[hashed(ids[0], 1000000)], table('age_embedding')[age]], 1)
-  item = torch.cat([table('item_id_embedding')[hashed(ids[2], V)], table('cate_id_embedding')[hashed(ids[3], 10000)],
-                    feats['dense_fea'] * table('price_embedding')[0][None, :]], 1)
-  lens = feats['seq_fea']['hist_items'][1]
-  mask = torch.arange(T, device=DEV)[None, :] < lens[:, None]
-  key = torch.cat([table('din/item_id_embedding')[hashed(ids[2], V)], table('din/cate_id_embedding')[hashed(ids[3], 10000)]], 1)
-  # the histories are STRING fields: they arrive host-hashed (input/readers.py), the slot is an identity lookup
-  he = torch.cat([table('din/hist_items_embedding')[feats['seq_fea']['hist_items'][0]],
-                  table('din/hist_cates_embedding')[feats['seq_fea']['hist_cates'][0]]], 2)
-  he = he * mask[:, :, None]
-  cur = key[:, None, :].expand(-1, T, -1)
-  din_in = torch.cat([cur, he, cur - he, cur * he], -1).reshape(B * T, -1)
-  scores = _dnn(model.din_dnn[0], din_in).reshape(B, 1, T)
-  scores = torch.where(mask[:, None, :], scores, torch.full_like(scores, -2.0**32 + 1))
-  att = (torch.softmax(scores, -1) @ he).reshape(B, -1)
-  feas = [_dnn(model.tower_dnn[0], _bn(user) * model.tower_bn[0].gamma + model.tower_bn[0].beta),
-          _dnn(model.tower_dnn[1], _bn(item) * model.tower_bn[1].gamma + model.tower_bn[1].beta),
-          torch.cat([att, key], 1)]
-  ref = (_dnn(model.final_dnn, torch.cat(feas, 1)) @ model.output.kernel + model.output.bias)[:, 0]
-  assert float((logits - ref).abs().max()) < 1e-4
-  # and a training step at this shape runs through the fused update (one arena: keys, histories, towers)
-  tr = est.trainer
-  labels = torch.from_numpy((np.random.default_rng(0).uniform(size=B) < 0.25).astype(np.float32)).to(DEV)
-  l0 = float(tr.train_step(feats, labels)[0])
-  for _ in range(5):
-    l1 = float(tr.train_step(feats, labels)[0])
-  assert np.isfinite(l0) and l1 < l0
-
-
-C5 = '''
-train_config { optimizer_config { adagrad_optimizer { learning_rate { constant_learning_rate { learning_rate: 0.02 } } } } }
-data_config { batch_size: %(B)d input_type: DummyInput label_fields: ["l0", "l1", "l2"] }
-feature_config {
-%(feats)s
-}
-model_config { model_class: "MultiTaskModel"
-  feature_groups { group_name: "all" feature_names: [%(names)s] wide_deep: DEEP }
-  backbone {
-    blocks { name: "deep" inputs { feature_group_name: "all" } keras_layer { class_name: "MLP" mlp { hidden_units: [256, 128] } } }
-    blocks { name: "cross" inputs { feature_group_name: "all" input_fn: "lambda x: [x, x]" }
-             recurrent { num_steps: 3 fixed_input_index: 0 keras_layer { class_name: "Cross" } } }
-    blocks { name: "both" inputs { block_name: "deep" } inputs { block_name: "cross" } merge_inputs_into_list: true
-             keras_layer { class_name: "Concatenate" } }
-    blocks { name: "mmoe" inputs { block_name: "both" }
-             keras_layer { class_name: "MMoE" mmoe { num_task: 3 num_expert: 4 expert_mlp { hidden_units: [128, 64] } } } }
-  }
-  model_params { l2_regularization: 1e-6
-    task_towers { tower_name: "t0" label_name: "l0" mlp { hidden_units: [64] } }
-    task_towers { tower_name: "t1" label_name: "l1" mlp { hidden_units: [64] } }
-    task_towers { tower_name: "t2" label_name: "l2" mlp { hidden_units: [64] } } }
-  embedding_regularization: 1e-6 }
-'''
-
-
-def test_c5_shaped_mmoe_over_cross_backbone_trains_and_mixes_like_the_oracle():
-  """C5: MMoE-3task on a DCN backbone, emb 32, batch 16384 (the 100M-row table scaled to 2M rows: one GPU test box)."""
-  torch.backends.cuda.matmul.allow_tf32 = False
-  B, n_f = 16384, 12
-  feats = '\n'.join('  features { input_names: "c%d" feature_type: IdFeature embedding_dim: 32 hash_bucket_size: 2000000 '
-                    'embedding_name: "shared" }' % i for i in range(n_f))
-  text = C5 % dict(B=B, feats=feats, names=', '.join('"c%d"' % i for i in range(n_f)))
-  try:
-    cfg = config_util.get_configs_from_pipeline_file(text.encode())
-    il, model, opt = builder.build_model(cfg, B, DEV, generator=torch.Generator(device=DEV).manual_seed(1),
-                                         cpu_generator=torch.Generator().manual_seed(1))
-  except NotImplementedError as e:
-    pytest.skip('config outside the scope check: %s' % e)
-  rng = np.random.default_rng(5)
-  ids = (rng.zipf(1.05, n_f * B).astype(np.int64) - 1) % (2**40)
-  f = {'sparse_fea': torch.from_numpy(ids).to(DEV)}
-  labels = torch.from_numpy((rng.uniform(size=(B, 3)) < 0.3).astype(np.float32)).to(DEV)
-  tr = Trainer(model, il, 'adagrad', lr_fn=opt['lr_fn'])
-  losses = [float(tr.train_step(f, labels)[0]) for _ in range(8)]
-  assert all(np.isfinite(losses)) and losses[-1] < losses[0]
-  # the mixture kernel against the oracle's layers/mmoe.py restatement on this batch's gate logits / expert outputs
-  from easyrec_b200 import interactions as I
-  g = torch.randn(B, 4, device=DEV)
-  ex = torch.randn(B, 4, 64, device=DEV)
-  got = I.mmoe_mix(g, ex).cpu().numpy()
-  p = np.exp(g.cpu().numpy() - g.cpu().numpy().max(1, keepdims=True))
-  p = p / p.sum(1, keepdims=True)
-  want = (p[:, :, None] * ex.cpu().numpy()).sum(1)
-  np.testing.assert_allclose(got, want, rtol=1e-5, atol=1e-5)
 
 
 TAG_CFG = b'''

@@ -940,10 +940,14 @@ def test_c5_workload_config_builds_and_trains_with_kernel_doubles(interaction_do
   """bench.py --workload mmoe_c5 (BASELINE.json configs[4]): the pipeline config text and the batch generator of
   easyrec_b200.workloads at a small size - MultiTaskModel over the Cross + MLP backbone, MMoE with 4 experts (the gate
   layers are the vector-sized GEMMs of er_gemm_small), three towers bound to their labels."""
-  from easyrec_b200 import workloads
+  from easyrec_b200 import layers as L, workloads
   from easyrec_b200.estimator import EasyRecEstimator
   est = EasyRecEstimator(workloads.c5_config_text(64, 5000, n_feat=6, embedding_parallel=False), device='cpu', seed=2)
   assert est.model.tower_names == ['t0', 't1', 't2'] and est.model.label_cols == [0, 1, 2]
+  # each task tower is the config's `dnn { hidden_units: [64] }` on the 64-wide MMoE output, then Dense(1)
+  for dnn, out in zip(est.model.tower_dnn, est.model.tower_out):
+    assert isinstance(dnn, L.DNN) and [tuple(l.kernel.shape) for l in dnn.layers] == [(64, 64)]
+    assert tuple(out.kernel.shape) == (64, 1)
   assert list(est.input_layer.arenas[32].tables) == ['shared'] and est.input_layer.arenas[32].n_rows == 5000
   feats, labels = workloads.c5_batch(64, 1, n_feat=6)
   assert feats['sparse_fea'].numel() == 6 * 64 and labels.shape == (64, 3)
